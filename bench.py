@@ -7,6 +7,7 @@ chi-square) followed by sample_spectral_parameters (Metropolis + chi-square).
 
   python bench.py --gpus N --steps K --warmup W          our arm (one process per GPU)
   python bench.py --impl reference ...                   the CPU oracle on the host cores
+  python bench.py ... --dump-outputs DIR                 also write the last timed step's outputs to DIR/*.npy
 
 The workload is BASELINE.json configs[1] ("c2": nside=512, 8 delta bands, Q+U, synch+dust, CG
 amplitudes + full-sky beta_d, NUMSAMPLE=20) on synthetic maps (dang_b200/synth.py).
@@ -160,6 +161,31 @@ def pinned_array(lib, shape):
     return np.frombuffer(buf, dtype=np.float64).reshape(shape)
 
 
+# ------------------------------------------------------------------ outputs of the timed path
+DUMP_BUDGET_BYTES = 60_000_000
+DUMP_SEED = 20260107
+
+
+def dump_outputs(out_dir, eng, cfg, n_cg, chisq):
+    """What the last timed Gibbs iteration left a caller: every component's amplitude maps [nmaps][npix] and index
+    maps [nind][nmaps][npix], the CG iteration count and the chi-square, as float64 .npy files.  When the maps exceed
+    the budget (60 MB in all), the same seeded, sorted sample of pixels is taken from every map (`pixels.npy` lists
+    it), so two builds run with the same arguments can be compared file by file."""
+    rows = sum(cfg.nmaps * (1 + len(c.indices)) for c in cfg.comps)
+    m = min(cfg.npix, DUMP_BUDGET_BYTES // (8 * (rows + 1)))
+    pix = np.arange(cfg.npix) if m == cfg.npix else np.sort(
+        np.random.default_rng(DUMP_SEED).choice(cfg.npix, size=m, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pixels": pix.astype(np.float64), "n_cg": np.array([n_cg], dtype=np.float64),
+              "chisq": np.array([chisq], dtype=np.float64)}
+    for ic, c in enumerate(cfg.comps):
+        arrays[f"amplitude_{c.label}"] = np.ascontiguousarray(eng.amplitude(ic)[:, pix])
+        if c.indices:
+            arrays[f"indices_{c.label}"] = np.ascontiguousarray(eng.indices(ic)[:, :, pix])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------ our arm
 def run_gpu(args):
     import torch
@@ -177,6 +203,8 @@ def run_gpu(args):
         torch.cuda.set_device(local)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     assert world == args.gpus or world == 1, (world, args.gpus)
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs: run a single process (each rank holds only its own pixels)")
 
     cfg = make_config(args.config, nside=args.nside)
     # big configs (nside >= 1024): every rank builds only its own pixel slice of the synthetic sky
@@ -274,6 +302,8 @@ def run_gpu(args):
     ms = max_over_ranks(eng.event_elapsed_ms(0, 1))
     launches = eng.launch_count()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:  # before the legs below move the chain on
+        dump_outputs(args.dump_outputs, eng, cfg, n_cg[-1], info["chisq"])
 
     # --- per-kernel timing for the roofline: same steps with CUDA events around every launch
     eng.kernel_stats(reset=True)
@@ -580,7 +610,13 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the reduced-traffic e2e variants")
     ap.add_argument("--defer-scalars", type=int, default=1, help="1: DANG_OPT_DEFER_SCALARS on the one-solve + full-sky configs")
     ap.add_argument("--opt", action="append", default=[], help="library option id=value (experiments), e.g. --opt 8=16")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's maps and scalars to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -29,8 +29,10 @@ def test_library_exports_every_declared_symbol():
 
 def test_library_is_sm100a_and_has_no_oracle_dependency():
     from dang_b200 import _lib
+    import shutil
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"  # build.sh's default toolkit, off PATH
+    out = subprocess.run([cuobjdump, "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     ldd = subprocess.run(["ldd", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "oracle" not in ldd

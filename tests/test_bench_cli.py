@@ -1,9 +1,12 @@
 """bench.py's CPU legs (no GPU): the reference arm prints one JSON line with the contract's keys, on rank 0 only
-under a multi-rank launch, and the product arm fails loudly without a device instead of falling back to the CPU."""
+under a multi-rank launch, and the product arm fails loudly without a device instead of falling back to the CPU.
+--dump-outputs is checked on a stub engine here and end to end on the GPU (marked `gpu`)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,6 +44,76 @@ def test_product_arm_has_no_cpu_fallback():
     r = _run(["--nside", "16", "--steps", "1", "--warmup", "1", "--no-cpu"])
     assert r.returncode != 0
     assert "dang_gpu" in (r.stderr + r.stdout) or "CUDA" in (r.stderr + r.stdout)
+
+
+def test_steps_and_dump_outputs_arguments_are_checked():
+    r = _run(["--impl", "reference", "--nside", "16", "--steps", "0"])
+    assert r.returncode == 2 and "--steps" in r.stderr
+    r = _run(["--impl", "reference", "--nside", "16", "--steps", "1", "--dump-outputs", "unused"])
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr
+
+
+class _StubEngine:
+    """amplitude / indices as Engine returns them, filled with values that encode (array, row, pixel)."""
+
+    def __init__(self, cfg):
+        import numpy as np
+        self.cfg, self.pix = cfg, np.arange(cfg.npix, dtype=np.float64)
+
+    def amplitude(self, ic):
+        import numpy as np
+        return np.stack([1e7 * ic + 1e6 * k + self.pix for k in range(self.cfg.nmaps)])
+
+    def indices(self, ic):
+        import numpy as np
+        nind = len(self.cfg.comps[ic].indices)
+        return np.stack([self.amplitude(ic) + 1e5 * (j + 1) for j in range(nind)])
+
+
+def test_dump_outputs_writes_a_fixed_sample_within_the_budget(tmp_path):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from dang_b200.synth import make_config
+    for nside, sampled in ((16, False), (512, True)):      # the bench workload at a small size and at its own size
+        cfg = make_config("c2", nside=nside)
+        dumps = []
+        for k in range(2):
+            d = tmp_path / f"n{nside}_{k}"
+            bench.dump_outputs(str(d), _StubEngine(cfg), cfg, 17, 1.25)
+            dumps.append({p.stem: np.load(p) for p in d.iterdir()})
+            assert sum(p.stat().st_size for p in d.iterdir()) <= 64_000_000
+        a, b = dumps
+        assert sorted(a) == ["amplitude_dust", "amplitude_synch", "chisq", "indices_dust", "indices_synch", "n_cg", "pixels"]
+        assert all(v.dtype == np.float64 for v in a.values())
+        assert all(np.array_equal(a[n], b[n]) for n in a)    # same arguments, same files
+        assert a["n_cg"].tolist() == [17.0] and a["chisq"].tolist() == [1.25]
+        pix = a["pixels"].astype(np.int64)
+        assert np.all(np.diff(pix) > 0) and (len(pix) < cfg.npix) == sampled
+        assert a["amplitude_dust"].shape == (cfg.nmaps, len(pix)) and a["indices_dust"].shape == (2, cfg.nmaps, len(pix))
+        assert np.array_equal(a["amplitude_dust"][2], 1e7 + 2e6 + pix)
+        assert np.array_equal(a["indices_synch"][0, 1], 1e6 + 1e5 + pix)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path_on_the_gpu(tmp_path):
+    """Same arguments, same outputs (also with the scalars read every step); one timed step more moves the chain on."""
+    import numpy as np
+
+    def dump(name, *extra, steps=3):
+        d = tmp_path / name
+        r = _run(["--nside", "16", "--steps", str(steps), "--warmup", "2", "--no-cpu", "--no-variants",
+                  "--dump-outputs", str(d), *extra], env={"DANG_BENCH_NO_CLOCKS": "1"})
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads([x for x in r.stdout.splitlines() if x.startswith("{")][-1])["steps"] == steps
+        return {p.stem: np.load(p) for p in d.iterdir()}
+
+    a, b, sync, more = dump("a"), dump("b"), dump("sync", "--defer-scalars", "0"), dump("more", steps=4)
+    assert sorted(a) == sorted(more) and len(a["pixels"]) == 3072 and 1 < a["n_cg"][0] < 100
+    for n in a:
+        assert np.array_equal(a[n], b[n]) and np.array_equal(a[n], sync[n]), n
+        assert np.all(np.isfinite(a[n])), n
+    assert not np.array_equal(a["amplitude_dust"], more["amplitude_dust"])
 
 
 def test_roofline_block_reports_the_bounding_pipe(monkeypatch):
