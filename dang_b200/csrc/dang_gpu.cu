@@ -951,6 +951,14 @@ int dang_gpu_get_cg_x(dang_gpu_t *h, int cg_group, int flag_n, double *x) {
   API_END
 }
 
+// Deferred scalars: the device keeps ONE full-sky draw's outcome (MhScalars) for dang_gpu_iteration_mark.  A second
+// full-sky draw -- or the tuner, which runs its chains in the same scalars -- before the mark would overwrite it.
+static void deferred_draw_guard(const dang_gpu *h) {
+  if (h->defer_scalars && h->pend_draw)
+    fail(DANG_GPU_ESTATE, "a deferred full-sky draw is pending: call dang_gpu_iteration_mark before the next full-sky "
+                          "draw or step-size tuning (its acceptance, value and chi-square would be lost)");
+}
+
 int dang_gpu_sample_index(dang_gpu_t *h, int ic, int nind, int map_n, int nsample, int ml_mode,
                           const double *z, const double *u, uint64_t seed, double *accept) {
   API_BEGIN
@@ -962,6 +970,7 @@ int dang_gpu_sample_index(dang_gpu_t *h, int ic, int nind, int map_n, int nsampl
     CK(cudaStreamWaitEvent(h->stream, h->ev_idx_dl, 0));
     h->idx_dl_pending = false;
   }
+  if (!perpix) deferred_draw_guard(h);
   h->fs_tab_written = false;
   if (perpix) {
     touch(h, 2);
@@ -1021,6 +1030,7 @@ int dang_gpu_tune_index(dang_gpu_t *h, int ic, int nind, int map_n, int nsample,
   if (nsample < 0) fail(DANG_GPU_EINVAL, "nsample = %d", nsample);
   MhView mh;
   mh_view(h, ic, nind, map_n, nsample, ml_mode, mh);
+  deferred_draw_guard(h);
   double start[DG_MAXIND] = {0.0, 0.0};
   const bool perpix = h->comp[ic].index[nind].index_mode == DANG_INDEX_PERPIXEL;
   if (perpix) {

@@ -371,7 +371,8 @@ mh_perpixel_fast_kernel(const __grid_constant__ ModelView mv, const __grid_const
           tr1[i] -= a1;
           g0[i] += a0;
           g1[i] += a1;
-          if (MODE == MH_SED_MBB_T) kj[i] = 1.0f + __frcp_rn(k5_em1f(cf[i * L] * iT));
+          // (padding bands keep K = 1: with c_j = 0, 1 / em1(0) would make every later proposal NaN)
+          if (MODE == MH_SED_MBB_T && r + i * L < B) kj[i] = 1.0f + __frcp_rn(k5_em1f(cf[i * L] * iT));
         }
         dT += kap * A1 + 1.2e-7f * (tmax + A2);       // error of a (b-scaled) + rounding of t - a
         kap += 1.5e-7f;                               // g picks up ~1 ulp per update
@@ -698,7 +699,7 @@ k5_chain_kernel(const __grid_constant__ ModelView mv, const __grid_constant__ Mh
           g0[i] += a0;
           g1[i] += a1;
           gs[i] = fabsf(g0[i]) + fabsf(g1[i]);
-          if (MODE == MH_SED_MBB_T) kj[i] = 1.0f + __frcp_rn(k5_em1f(cf[i] * iT));
+          if (MODE == MH_SED_MBB_T && r + i * L < B) kj[i] = 1.0f + __frcp_rn(k5_em1f(cf[i] * iT));  // (padding: K = 1)
         }
         dT += kap * A1 + 1.2e-7f * (tmax + A2);
         kap += 1.5e-7f;

@@ -300,7 +300,10 @@ int dang_gpu_udgrade(dang_gpu_t *h, int kind, const double *in, int nside_in, do
 /* ---- deferred scalars (DANG_OPT_DEFER_SCALARS): the terminal line of src/dang.f90:100-104 one iteration late ----
  * _mark: snapshot what the deferred calls since the previous mark left on the device (solve count / residual,
  *   statistics rows, chain outcome) into one of four pinned slots, stream ordered, no host wait; returns a ticket.
- *   At most four tickets may be outstanding (unread).
+ *   At most four tickets may be outstanding (unread).  A slot holds ONE full-sky draw: a second full-sky
+ *   dang_gpu_sample_index (or a dang_gpu_tune_index) before the next _mark would overwrite the first draw's outcome
+ *   and fails with DANG_GPU_ESTATE instead -- mark after each full-sky draw (index poltype 'Q,U', or several
+ *   full-sky indices per iteration).
  * _scalars: wait for that snapshot only and decode it.  n_iter / delta_final: the amplitude draw's (as
  *   dang_gpu_cg_solve); chisq_after_amplitudes[nmaps]: the dang_gpu_chisq call that followed it; accept /
  *   index_value: the full-sky draw's acceptance ratio and final value; chisq_after_index[nmaps]: the dang_gpu_chisq

@@ -31,6 +31,10 @@ def main():
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     worst = 0.0
     ns = int(os.environ.get("DANG_MGC_NSIDE", "16"))
+    if os.environ.get("DANG_MGC_CASE") == "b32":
+        check_32_bands(rank, world, local, ns)
+        dist.destroy_process_group()
+        return
     from dang_b200.engine import OPT_CG_CHECKPOINT
     # (config, nside, CG form): the default checkpointed-recompute form, the streaming form (checkpoint 0) and a
     # solve with i_max >= DG_CG_HIST (1024), which also takes the streaming form -- all exchange the CG sums
@@ -137,6 +141,43 @@ def main():
             assert np.array_equal(a, b), (rank, "deferred-scalars maps differ")
     print(f"rank {rank}/{world}: multi-GPU parity ok (pixels [{lo},{hi}), worst amplitude error {worst:.2e})", flush=True)
     dist.destroy_process_group()
+
+
+def check_32_bands(rank, world, local, nside):
+    """DANG_MGC_CASE=b32: full-sky draws at 32 bands (S = 2, then S = 1 on Q), whose statistics rows of
+    3 x 4 x 8 chunks x S values per rank are the largest the scalar exchange carries."""
+    import torch.distributed as dist
+
+    from dang_b200.engine import Engine, setup_torch_comm
+    from dang_b200.healpix import ring_partition
+    from oracle.binding import Oracle
+    from test_gpu_shapes import shape_case
+    cfg, sky = shape_case(32, nside=nside, varying=())
+    spec = cfg.comps[1].indices[0]
+    spec.sample, spec.region, spec.step = True, "fullsky", 0.002
+    bounds = ring_partition(cfg.nside, world, weights=(sky.mask != 0).astype(np.float64))
+    lo, hi = int(bounds[rank]), int(bounds[rank + 1])
+    eng = Engine(cfg, sky, device=local, pix_range=(lo, hi))
+    setup_torch_comm(eng, mailboxes=os.environ.get("DANG_GPU_MAILBOX", "1") != "0")
+    ora = Oracle(cfg, sky)
+    rng = np.random.default_rng(79)
+    for map_n, nsample in ((-1, 24), (2, 200)):
+        z, u = rng.standard_normal(nsample), rng.random(nsample)
+        acc_o, dec_o, lnl_o = ora.sample_index_mh(1, 0, map_n, nsample, 1, z, u, want_trace=True)
+        acc_g = eng.sample_index_mh(1, 0, map_n, nsample, "sample", z, u)
+        dec_g, lnl_g = eng.decisions(nsample, fullsky=True)
+        assert np.array_equal(dec_g, dec_o[:nsample]) and acc_g == acc_o, (rank, map_n, dec_g, dec_o[:nsample])
+        ev = dec_o[:nsample] < 2
+        assert np.max(np.abs(lnl_g[ev] - lnl_o[:nsample][ev])) <= 1e-10 * np.max(np.abs(lnl_o[:nsample][ev])), (rank, map_n)
+        ia, ib = eng.indices(1)[:, :, lo:hi], ora.indices(1)[:, :, lo:hi]
+        assert np.max(np.abs(ia - ib)) <= 1e-14 * np.max(np.abs(ib)), (rank, map_n)
+        ora.update_sky_model()
+        chisq_o, _ = ora.compute_chisq()
+        assert abs(eng.compute_chisq() - chisq_o) <= 1e-10 * chisq_o, (rank, map_n)
+    eng.comm_check()
+    eng.close()
+    dist.barrier()
+    print(f"rank {rank}/{world}: multi-GPU parity ok (32 bands, pixels [{lo},{hi}))", flush=True)
 
 
 if __name__ == "__main__":

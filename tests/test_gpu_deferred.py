@@ -96,3 +96,16 @@ def test_deferred_mode_is_loud_about_misuse():
     with pytest.raises(DangGpuError, match="overwritten"):
         eng.iteration_scalars(t[0])
     assert eng.iteration_scalars(t5)["n_iter"] > 1
+    # a mark holds one full-sky outcome: a second full-sky draw before it (index poltype 'Q,U', or two full-sky
+    # indices in one iteration) would overwrite the first draw's acceptance, value and chi-square
+    eng.sample_index_mh(1, 0, 2, 8, seed=4)
+    with pytest.raises(DangGpuError, match="iteration_mark"):
+        eng.sample_index_mh(1, 0, 3, 8, seed=4)
+    with pytest.raises(DangGpuError, match="iteration_mark"):
+        eng.tune_index(1, 0, 3, 8, seed=4, max_blocks=2)
+    t6 = eng.iteration_mark()
+    eng.sample_index_mh(1, 0, 3, 8, seed=4)
+    t7 = eng.iteration_mark()
+    s6, s7 = eng.iteration_scalars(t6), eng.iteration_scalars(t7)
+    assert s6["index_value"] == eng.index_fullsky(1, 0, 2) and s7["index_value"] == eng.index_fullsky(1, 0, 3)
+    assert s6["accept"] >= 0.0 and s7["accept"] >= 0.0  # (NaN: nothing was snapshot)
