@@ -35,6 +35,10 @@ def main():
         check_32_bands(rank, world, local, ns)
         dist.destroy_process_group()
         return
+    if os.environ.get("DANG_MGC_CASE") == "rng":
+        check_device_deviates(rank, world, local, ns)
+        dist.destroy_process_group()
+        return
     from dang_b200.engine import OPT_CG_CHECKPOINT
     # (config, nside, CG form): the default checkpointed-recompute form, the streaming form (checkpoint 0) and a
     # solve with i_max >= DG_CG_HIST (1024), which also takes the streaming form -- all exchange the CG sums
@@ -178,6 +182,47 @@ def check_32_bands(rank, world, local, nside):
     eng.close()
     dist.barrier()
     print(f"rank {rank}/{world}: multi-GPU parity ok (32 bands, pixels [{lo},{hi}))", flush=True)
+
+
+def check_device_deviates(rank, world, local, nside):
+    """DANG_MGC_CASE=rng: Gibbs iterations with the device's own deviates, as bench.py runs them -- c2 (full-sky beta_d,
+    tuned once) and c1 (per-pixel beta_s).  Every rank draws its pixels' eta and z / u at global slots, so its slice
+    must follow the single-process oracle fed the Philox arrays (tests/test_gpu_device_rng.py)."""
+    import torch.distributed as dist
+
+    from dang_b200.engine import Engine, setup_torch_comm
+    from dang_b200.healpix import ring_partition
+    from helpers import small_case
+    from oracle.binding import Oracle
+    from test_gpu_device_rng import oracle_gibbs_iteration
+    seed = 9
+    for name, ns in (("c2", nside), ("c1", 16)):
+        cfg, sky = small_case(name, ns, perturb=False)
+        if name == "c2":
+            cfg.comps[1].indices[0].tune = True
+        bounds = ring_partition(cfg.nside, world, weights=(sky.mask != 0).astype(np.float64))
+        lo, hi = int(bounds[rank]), int(bounds[rank + 1])
+        eng = Engine(cfg, sky, device=local, pix_range=(lo, hi))
+        setup_torch_comm(eng, mailboxes=os.environ.get("DANG_GPU_MAILBOX", "1") != "0")
+        ora = Oracle(cfg, sky)
+        tuned = [[not s.tune for s in c.indices] for c in cfg.comps]
+        for it in range(1, 5):
+            n_o, chi_cg_o, acc_o, chi_mh_o, _ = oracle_gibbs_iteration(ora, cfg, it, seed, tuned)
+            r1, r2 = eng.gibbs_iteration(it, seed=seed)
+            assert r1[0][0] == n_o[0], (rank, name, it, r1[0][0], n_o)
+            assert abs(r1[1] - chi_cg_o) <= 1e-10 * chi_cg_o, (rank, name, it, r1[1], chi_cg_o)
+            if it > 1:
+                assert r2[0] == acc_o, (rank, name, it, r2[0], acc_o)
+                assert abs(r2[1] - chi_mh_o) <= 1e-10 * chi_mh_o, (rank, name, it, r2[1], chi_mh_o)
+            for ic in range(len(cfg.comps)):
+                a, b = eng.amplitude(ic)[:, lo:hi], ora.amplitude(ic)[:, lo:hi]
+                assert np.max(np.abs(a - b)) <= 1e-10 * np.max(np.abs(ora.amplitude(ic))), (rank, name, it, ic)
+                ia, ib = eng.indices(ic)[:, :, lo:hi], ora.indices(ic)[:, :, lo:hi]
+                assert np.max(np.abs(ia - ib)) <= 1e-14 * np.max(np.abs(ib)), (rank, name, it, ic)
+        eng.comm_check()
+        eng.close()
+        dist.barrier()
+    print(f"rank {rank}/{world}: multi-GPU parity ok (device deviates, pixels [{lo},{hi}))", flush=True)
 
 
 if __name__ == "__main__":

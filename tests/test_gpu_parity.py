@@ -183,7 +183,9 @@ def test_cg_recovers_noiseless_sky():
 
 def test_device_rng_eta_matches_philox_definition():
     """eta == NULL: the device draws eta from Philox4x32-10; feeding the oracle the same stream
-    (restated independently in oracle/dang_oracle.c) gives the same amplitudes."""
+    (restated independently in oracle/dang_oracle.c) gives the same amplitudes.  The device's normals are
+    r * sinpi(2 u2), the oracle's r * sin(2 pi u2): they differ by an ulp or so, and the amplitudes stay within
+    TOL (~7e-16 measured on a B200; tests/test_gpu_device_rng.py covers every other call site)."""
     from oracle.binding import philox_normals
     cfg, sky, ora, eng = make_pair("c1", 8)
     seed = 1234567
@@ -193,7 +195,7 @@ def test_device_rng_eta_matches_philox_definition():
     it_g, _ = eng.cg_solve(0, 0, "sample", eta=None, seed=seed)
     assert it_g == it_o
     for ic in range(2):
-        assert rel_err(eng.amplitude(ic), ora.amplitude(ic)) < 1e-9
+        assert rel_err(eng.amplitude(ic), ora.amplitude(ic)) < TOL
 
 
 # ------------------------------------------------------------------ spectral-parameter draw
