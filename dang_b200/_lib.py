@@ -67,6 +67,7 @@ SIGNATURES = {
     "dang_gpu_download_wait": (C.c_int, [vp]),
     "dang_gpu_stage_eta": (C.c_int, [vp, c_dp, C.c_int]),
     "dang_gpu_bandpass_quadrature": (C.c_int, [C.c_double, C.c_int, c_dp, c_dp, C.c_int, c_dp, c_dp]),
+    "dang_gpu_band_samples": (C.c_int, [vp, C.c_int, c_ip]),
     "dang_gpu_host_alloc": (C.c_int, [C.POINTER(vp), C.c_uint64]),
     "dang_gpu_host_free": (C.c_int, [vp]),
     "dang_gpu_event_record": (C.c_int, [vp, C.c_int]),

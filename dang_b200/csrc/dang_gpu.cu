@@ -36,10 +36,13 @@ void nccl_load() {
 // x = ln(nu / nu_c) over the few per cent a band spans.  The n-point Gauss rule of the discrete measure
 // {x_i, tau0_i} -- nodes = eigenvalues of its Jacobi matrix (Lanczos on diag(x) started from sqrt(tau0)),
 // weights = total weight x squared first eigenvector components -- integrates every polynomial in x up to
-// degree 2n-1 exactly as the full table does, so for n = 8 the two sums differ by the 16th-order Taylor
-// remainder of g across the band: < 1e-17 relative for power-law / Planck factors over a 30 % band, far
-// below the rounding of the n_bp-term sum.  The device then sees n samples per band instead of n_bp (128 at
-// config c3): 16x fewer transcendentals in every kernel that evaluates a bandpass-integrated SED.
+// degree 2n-1 exactly as the full table does, so the two sums differ by the 2n-th order Taylor remainder of g
+// across the band.  That remainder is below rounding only while g varies slowly in ln nu: it is for power laws
+// and mbb dust at the c3 bands, but not for 'cmb' above ~500 GHz (hnu/kT_CMB up to 15 at 857 GHz: 4e-8 with 8
+// nodes over a half-width of 0.25) or for a narrow lognormal near nu_p (2e-6 at w = 0.1).  So upload_bandpasses
+// accepts a rule for a band only after verifying it (verify_rule) and otherwise keeps the table.  With a rule
+// the device sees n samples per band instead of n_bp (128 at config c3): 16x fewer transcendentals in every
+// kernel that evaluates a bandpass-integrated SED.
 // Returns false (table kept) if the band is too short, has negative weights, or the rule comes out badly.
 static bool gauss_compress(const BandHost &b, int nq, std::vector<double> &nu_q, std::vector<double> &w_q) {
   std::vector<double> x, w;
@@ -133,6 +136,122 @@ static bool gauss_compress(const BandHost &b, int nq, std::vector<double> &nu_q,
   return fabsl(wsum - (long double)W) <= 1e-12L * (long double)W;
 }
 
+// Verification of a band's rule.  The values of an index a kernel can evaluate an SED at: the range of the maps
+// the host uploaded and, when the index is sampled, its uniform-prior box (the samplers never leave it).
+static void index_box(const dang_gpu *h, const CompHost &c, int l, double box[2]) {
+  box[0] = c.map_range[l][0];
+  box[1] = c.map_range[l][1];
+  if (c.index[l].sample_index) {
+    box[0] = std::min(box[0], c.index[l].uni[0]);
+    box[1] = std::max(box[1], c.index[l].uni[1]);
+  }
+}
+// the T_CMB values the 'cmb' SED can see: the current one and every value a 'T_cmb' component can hand over
+static void t_cmb_box(const dang_gpu *h, double box[2]) {
+  box[0] = box[1] = h->T_cmb;
+  for (int c = 0; c < h->ncomp; c++)
+    if (h->comp[c].set && h->comp[c].type == DANG_COMP_T_CMB) {
+      double b[2];
+      index_box(h, h->comp[c], 0, b);
+      box[0] = std::min(box[0], b[0]);
+      box[1] = std::max(box[1], b[1]);
+    }
+}
+// c%indices(:,:,l) as the host uploads it (full-sky [plane][pix], NULL: the constructor's 1.0): its range here
+static void record_map_range(const dang_gpu *h, CompHost &c, int l, const double *indices) {
+  double lo = 1.0, hi = 1.0;
+  if (indices) {
+    lo = INFINITY;
+    hi = -INFINITY;
+    for (int k = 0; k < h->nmaps; k++)
+      for (int64_t p = h->lo; p < h->hi; p++) {
+        const double v = indices[(size_t)k * h->npix + p];
+        lo = std::min(lo, v);
+        hi = std::max(hi, v);
+      }
+  }
+  c.map_range[l][0] = lo;
+  c.map_range[l][1] = hi;
+}
+// true while every index map and T_CMB stays inside the box the current rules were verified on
+static bool rules_cover_params(const dang_gpu *h) {
+  double box[2];
+  for (int c = 0; c < h->ncomp; c++)
+    for (int l = 0; h->comp[c].set && l < h->comp[c].nind; l++) {
+      index_box(h, h->comp[c], l, box);
+      if (!(box[0] >= h->comp[c].verified_box[l][0] && box[1] <= h->comp[c].verified_box[l][1])) return false;
+    }
+  t_cmb_box(h, box);
+  return box[0] >= h->verified_T_cmb[0] && box[1] <= h->verified_T_cmb[1];
+}
+// A band's SED up to factors constant over the band, in long double: the bodies of sed_powerlaw ... sed_planck_rj
+// (common.cuh), which restate evaluate_powerlaw ... evaluate_hi_fit of the reference.  hi_fit's template amplitude
+// and T_cmb's / hi_fit's constants cancel in a relative comparison.
+static long double sed_ld(int type, long double nu, long double nu_ref, long double t0, long double t1, long double T_cmb) {
+  const long double H = (long double)DG_H, KB = (long double)DG_KB;
+  switch (type) {
+    case DANG_COMP_POWERLAW: return powl(nu / nu_ref, t0);
+    case DANG_COMP_MBB: return powl(nu / nu_ref, t0 + 1.0L) / expm1l(H * nu / (KB * t1));
+    case DANG_COMP_FREEFREE: {
+      const long double g = logl(expl(5.960L - sqrtl(3.0L) / 3.141592653589793238462643383279502884L *
+                                                  logl(nu / 1e9L * powl(t0 / 1e4L, -1.5L))) + 2.71828L);
+      return g * (nu_ref / nu) * (nu_ref / nu);
+    }
+    case DANG_COMP_LOGNORMAL: {
+      const long double t = logl(nu / (t0 * 1e9L)) / t1;
+      return expl(-0.5L * t * t) * (nu_ref / nu) * (nu_ref / nu);
+    }
+    case DANG_COMP_CMB: {
+      const long double y = (nu > 1e7L ? H * nu : H * nu * 1e9L) / (KB * T_cmb);
+      return expm1l(y) * expm1l(y) / (y * y * expl(y));
+    }
+    default: return nu / expm1l(H * nu / (KB * t0));  // T_cmb, hi_fit: B_nu / RJ
+  }
+}
+const int DG_VERIFY_POINTS = 7;  // per index dimension, box edges included
+// One point at which a band's rule is verified: an SED type and its parameters, with the full table's sum there.
+struct VerifyPoint {
+  int type;
+  long double nu_ref, t0, t1, full;
+};
+// The points for band b: for every component on the handle, a DG_VERIFY_POINTS grid over the box each of its indices
+// can take (a single point where the box is), each with sum_i tau0_i g(nu0_i) over the whole table.
+static std::vector<VerifyPoint> verify_points(const dang_gpu *h, const BandHost &b) {
+  std::vector<VerifyPoint> pts;
+  const int P = DG_VERIFY_POINTS;
+  for (int c = 0; c < h->ncomp; c++) {
+    const CompHost &cc = h->comp[c];
+    if (!cc.set || cc.type == DANG_COMP_TEMPLATE || cc.type == DANG_COMP_MONOPOLE) continue;
+    double box[2][2] = {{0.0, 0.0}, {0.0, 0.0}};  // 'cmb': box[0] is the T_CMB range
+    if (cc.type == DANG_COMP_CMB) t_cmb_box(h, box[0]);
+    for (int l = 0; l < cc.nind; l++) index_box(h, cc, l, box[l]);
+    const int n0 = box[0][1] > box[0][0] ? P : 1, n1 = box[1][1] > box[1][0] ? P : 1;
+    for (int a = 0; a < n0; a++)
+      for (int e = 0; e < n1; e++) {
+        VerifyPoint v;
+        v.type = cc.type;
+        v.nu_ref = cc.nu_ref;
+        v.t0 = box[0][0] + (box[0][1] - box[0][0]) * (long double)a / (P - 1);
+        v.t1 = box[1][0] + (box[1][1] - box[1][0]) * (long double)e / (P - 1);
+        v.full = 0.0L;
+        for (int i = 0; i < b.n; i++)
+          if (b.nu0[i] != 0.0) v.full += (long double)b.tau0[i] * sed_ld(v.type, b.nu0[i], v.nu_ref, v.t0, v.t1, v.t0);
+        pts.push_back(v);
+      }
+  }
+  return pts;
+}
+// Does the rule (nu_q, w_q) reproduce the table's sum to 1e-14 relative at every point?
+static bool verify_rule(const std::vector<VerifyPoint> &pts, const std::vector<double> &nu_q,
+                        const std::vector<double> &w_q) {
+  for (const VerifyPoint &v : pts) {
+    long double q = 0.0L;
+    for (size_t k = 0; k < nu_q.size(); k++) q += (long double)w_q[k] * sed_ld(v.type, nu_q[k], v.nu_ref, v.t0, v.t1, v.t0);
+    if (!(fabsl(q - v.full) <= 1e-14L * fabsl(v.full))) return false;
+  }
+  return true;
+}
+
 void upload_bandpasses(dang_gpu *h) {
   if (!h->bp_dirty) return;
   std::vector<double> nu0, tau0;
@@ -141,17 +260,25 @@ void upload_bandpasses(dang_gpu *h) {
     b.n_dev = b.n;
     b.nu0_dev = b.nu0;
     b.tau0_dev = b.tau0;
-    if (h->bp_quad > 0 && b.n > 0) {
+    // the smallest rule (bp_quad, then 4 nodes more at a time, up to n_bp / 2) that verify_rule accepts
+    std::vector<VerifyPoint> pts;
+    if (h->bp_quad > 0 && 2 * h->bp_quad <= b.n) pts = verify_points(h, b);
+    for (int nq = h->bp_quad; nq > 0 && 2 * nq <= b.n; nq += 4) {
       std::vector<double> nq_nu, nq_w;
-      if (gauss_compress(b, h->bp_quad, nq_nu, nq_w)) {
-        b.n_dev = h->bp_quad;
+      if (!gauss_compress(b, nq, nq_nu, nq_w)) break;
+      if (verify_rule(pts, nq_nu, nq_w)) {
+        b.n_dev = nq;
         b.nu0_dev = nq_nu;
         b.tau0_dev = nq_w;
+        break;
       }
     }
     nu0.insert(nu0.end(), b.nu0_dev.begin(), b.nu0_dev.end());
     tau0.insert(tau0.end(), b.tau0_dev.begin(), b.tau0_dev.end());
   }
+  for (int c = 0; c < h->ncomp; c++)
+    for (int l = 0; h->comp[c].set && l < h->comp[c].nind; l++) index_box(h, h->comp[c], l, h->comp[c].verified_box[l]);
+  t_cmb_box(h, h->verified_T_cmb);
   dfree(h->bp_nu0); dfree(h->bp_tau0); dfree(h->bp_lnr_hi); dfree(h->bp_lnr_lo);
   h->nbp = (int)nu0.size();
   std::vector<double> lhi((size_t)h->ncomp * h->nbp + 1), llo((size_t)h->ncomp * h->nbp + 1);
@@ -746,6 +873,7 @@ int dang_gpu_set_component(dang_gpu_t *h, int ic, int type, const char *label, d
     fill_kernel<<<h->num_sms * 2, DG_THREADS, 0, h->stream>>>(c.idx[l], (int64_t)n2, 1.0);
     CK(cudaGetLastError());
     if (indices) h2d_planes(h, c.idx[l], indices + (size_t)l * h->nmaps * h->npix, h->nmaps);
+    record_map_range(h, c, l, indices ? indices + (size_t)l * h->nmaps * h->npix : nullptr);
   }
   for (int l = 0; l < DG_MAXIND; l++) {
     c.index[l] = IndexHost();
@@ -795,6 +923,7 @@ int dang_gpu_set_t_cmb(dang_gpu_t *h, double t_cmb) {
   if (!(t_cmb > 0.0)) fail(DANG_GPU_EINVAL, "T_CMB = %g", t_cmb);
   h->T_cmb = t_cmb;
   h->tab_dirty = true;  // the 'cmb' SED (1 / a2t) depends on it
+  if (!rules_cover_params(h)) h->bp_dirty = true;
   touch(h);
   API_END
 }
@@ -829,6 +958,7 @@ int dang_gpu_set_index(dang_gpu_t *h, int ic, int nind, int sample_index, int in
   ix.sample_nside = sample_nside;
   ix.nflag = nflag;
   for (int k = 0; k < nflag; k++) ix.pol_flag[k] = pol_flags[k];
+  if (!rules_cover_params(h)) h->bp_dirty = true;  // a wider prior box: verify the bandpass rules again
   touch(h);
   API_END
 }
@@ -846,10 +976,13 @@ int dang_gpu_set_amplitude(dang_gpu_t *h, int ic, const double *amplitude) {
 int dang_gpu_set_indices(dang_gpu_t *h, int ic, const double *indices) {
   API_BEGIN
   if (ic < 0 || ic >= h->ncomp || !h->comp[ic].set || !indices) fail(DANG_GPU_EINVAL, "bad component %d", ic);
-  for (int l = 0; l < h->comp[ic].nind; l++)
+  for (int l = 0; l < h->comp[ic].nind; l++) {
     h2d_planes(h, h->comp[ic].idx[l], indices + (size_t)l * h->nmaps * h->npix, h->nmaps);
+    record_map_range(h, h->comp[ic], l, indices + (size_t)l * h->nmaps * h->npix);
+  }
   CK(cudaStreamSynchronize(h->stream));
   h->tab_dirty = true;
+  if (!rules_cover_params(h)) h->bp_dirty = true;  // values outside the box the bandpass rules were verified on
   touch(h);
   for (int k = 0; k < 3; k++)
     for (int l = 0; l < DG_MAXIND; l++) h->check_mask |= 1ull << ((ic * 3 + k) * DG_MAXIND + l);
@@ -1354,6 +1487,14 @@ int dang_gpu_bandpass_quadrature(double nu_c_hz, int n_bp, const double *nu0_hz,
     w_q[k] = w[k];
   }
   return DANG_GPU_OK;
+}
+
+int dang_gpu_band_samples(dang_gpu_t *h, int band, int *n_samples) {
+  API_BEGIN
+  if (band < 0 || band >= h->nbands || !h->band[band].set || !n_samples) fail(DANG_GPU_EINVAL, "bad band %d", band);
+  upload_bandpasses(h);
+  *n_samples = h->band[band].n_dev;
+  API_END
 }
 
 int dang_gpu_host_alloc(void **ptr, uint64_t bytes) {

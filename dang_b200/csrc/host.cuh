@@ -106,6 +106,10 @@ struct CompHost {
   bool read_pending = false, read_pending_alt = false;
   double *idx[DG_MAXIND] = {nullptr, nullptr};
   IndexHost index[DG_MAXIND];
+  // range of the index maps the host last uploaded (this handle's pixels), and the box of index values the
+  // bandpass rules were verified on (upload_bandpasses)
+  double map_range[DG_MAXIND][2] = {{1.0, 1.0}, {1.0, 1.0}};
+  double verified_box[DG_MAXIND][2] = {{0.0, -1.0}, {0.0, -1.0}};
 };
 
 struct CgGroupHost {
@@ -206,6 +210,7 @@ struct dang_gpu {
   double *bp_nu0 = nullptr, *bp_tau0 = nullptr, *bp_lnr_hi = nullptr, *bp_lnr_lo = nullptr;
   int nbp = 0;
   bool bp_dirty = true;   // band / component constants changed: rebuild the static tables
+  double verified_T_cmb[2] = {0.0, -1.0};  // T_CMB range the 'cmb' SED was verified on
   bool tab_dirty = true;  // an index map changed: re-tabulate SEDs
   unsigned long long check_mask = ~0ull;  // index maps whose uniformity must be re-scanned
   SedTable *tab = nullptr;

@@ -292,6 +292,13 @@ module dang_gpu_mod
        integer(c_int), value :: ic, nind
        real(c_double) :: step_size
      end function dang_gpu_get_step_size
+     ! ---- samples of bp(band) the device sums over: 0 delta, n_bp table, else the verified Gauss rule's nodes
+     integer(c_int) function dang_gpu_band_samples(h, band, n_samples) bind(C, name='dang_gpu_band_samples')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: h
+       integer(c_int), value :: band
+       integer(c_int) :: n_samples
+     end function dang_gpu_band_samples
      ! ---- deferred scalars (DANG_OPT_DEFER_SCALARS = 18): the numbers of write_stats_to_term (dang.f90:100-104)
      !      one iteration late; a host that prints every iteration calls _mark at the end of iteration k and
      !      _scalars(ticket of k-1) right after it

@@ -113,10 +113,11 @@ enum {
   DANG_OPT_PERPIXEL_BP_SERIES = 13,
   /* Tabulated bandpasses are handed to the device as the n-point Gauss quadrature of the discrete measure
    * {ln(nu0_i / nu_c), tau0_i} (default n = 8; 0: the table itself).  The rule reproduces the table's sum for
-   * every polynomial in ln nu up to degree 2n-1, so bandpass-integrated SEDs agree with the n_bp-term sums of
-   * evaluate_powerlaw / evaluate_mbb / ... to < 1e-15 relative while costing n instead of n_bp
-   * transcendentals per band (DESIGN.md 4.2).  Bands with n_bp <= 2n, negative weights or a half-width above 0.25 in
-   * ln(nu) keep their table. */
+   * every polynomial in ln nu up to degree 2n-1 while costing n instead of n_bp transcendentals per band
+   * (DESIGN.md 4.2).  A band gets a rule only where it reproduces the n_bp-term sums of evaluate_powerlaw /
+   * evaluate_mbb / ... of every component on the handle to 1e-14 relative (n, n + 4, ... nodes are tried up to
+   * n_bp / 2; dang_gpu_band_samples reports the outcome).  Bands with negative weights or a half-width above 0.25 in
+   * ln(nu), and bands no rule passes for, keep their table. */
   DANG_OPT_BP_QUADRATURE = 14,
   /* 1 (default): the whole loop of cg_search (src/dang_cg_mod.f90:293-314) runs as ONE persistent, cooperatively
    * launched kernel -- one sweep of the checkpointed-recompute form per CG iteration, a grid barrier and (on
@@ -334,10 +335,18 @@ int dang_gpu_stage_eta(dang_gpu_t *h, const double *eta, int nplanes);
 
 /* The n-point Gauss quadrature the library substitutes for a tabulated bandpass (DANG_OPT_BP_QUADRATURE):
  * nodes nu_q [Hz] and weights w_q with sum_q w_q g(nu_q) == sum_i tau0_i g(nu0_i) for every g polynomial in
- * ln(nu) up to degree 2 nq - 1.  Host-only (no device needed); DANG_GPU_EUNSUPPORTED when the library would keep
- * the table (n_bp <= 2 nq, negative weights, half-width above 0.25 in ln nu). */
+ * ln(nu) up to degree 2 nq - 1.  Host-only (no device needed); DANG_GPU_EUNSUPPORTED when no rule is built
+ * (n_bp <= 2 nq, negative weights, half-width above 0.25 in ln nu).  This is the rule before a handle verifies it
+ * against its components' SEDs (dang_gpu_band_samples). */
 int dang_gpu_bandpass_quadrature(double nu_c_hz, int n_bp, const double *nu0_hz, const double *tau0, int nq,
                                  double *nu_q_hz, double *w_q);
+/* Samples of `band` that the device's bandpass-integrated SEDs sum over: 0 for a delta band, n_bp where the
+ * table is kept, otherwise the node count of the Gauss rule that replaced it.  A rule is used only where it
+ * reproduces the table's sum of every SED on the handle to 1e-14 relative at 7 points per index spanning the
+ * uniform-prior box of each sampled index and the range of the index maps uploaded (and at the T_CMB values 'cmb'
+ * can meet) -- a sampled check, not a bound between the points; it has DANG_OPT_BP_QUADRATURE nodes, or 4, 8, ...
+ * more (up to n_bp / 2) where that is not enough.  Read-only. */
+int dang_gpu_band_samples(dang_gpu_t *h, int band, int *n_samples);
 
 /* ---- instrumentation (bench.py) ---- */
 int dang_gpu_host_alloc(void **ptr, uint64_t bytes); /* pinned host memory */
