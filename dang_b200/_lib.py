@@ -79,6 +79,11 @@ SIGNATURES = {
     "dang_gpu_set_t_cmb": (C.c_int, [vp, C.c_double]),
     "dang_gpu_udgrade": (C.c_int, [vp, C.c_int, c_dp, C.c_int, c_dp, C.c_int, C.c_int, C.c_double]),
     "dang_gpu_comm_probe": (C.c_int, [vp, C.c_int, C.c_int, c_dp]),
+    "dang_gpu_posterior_begin": (C.c_int, [vp, C.c_int, C.c_int, C.c_int]),
+    "dang_gpu_posterior_accumulate": (C.c_int, [vp]),
+    "dang_gpu_posterior_get": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, c_dp, c_dp, c_i64p]),
+    "dang_gpu_posterior_end": (C.c_int, [vp]),
+    "dang_gpu_posterior_rhat": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, c_dp]),
 }
 
 _lib = None

@@ -8,7 +8,7 @@ obj="$here/_obj"
 mkdir -p "$obj"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-std=c++17 -O3 -lineinfo -gencode arch=compute_100a,code=sm_100a -Xcompiler -fPIC,-O2,-Wall "$@")
-units=(dang_gpu host_cg host_tmpl host_data host_mh_pp host_mh_ppd2 host_mh_ppd3 host_mh_ppd5 host_mh_ppd8 host_mh_ppf host_mh_ppx host_mh_fs host_udgrade)
+units=(dang_gpu host_cg host_tmpl host_data host_mh_pp host_mh_ppd2 host_mh_ppd3 host_mh_ppd5 host_mh_ppd8 host_mh_ppf host_mh_ppx host_mh_fs host_udgrade host_post)
 declare -A deps=(
   [dang_gpu]="kernels_data.cuh"
   [host_cg]="kernels_cg.cuh kernels_cg_solve.cuh kernels_uni.cuh kernels_stream.cuh"
@@ -17,6 +17,7 @@ declare -A deps=(
   [host_mh_pp]="kernels_mh.cuh"
   [host_mh_ppf]="kernels_mh.cuh kernels_mh_fast.cuh"
   [host_udgrade]=""
+  [host_post]="kernels_post.cuh kernels_data.cuh"
   [host_mh_ppd2]="kernels_mh.cuh host_mh_ppd.inc"
   [host_mh_ppd3]="kernels_mh.cuh host_mh_ppd.inc"
   [host_mh_ppd5]="kernels_mh.cuh host_mh_ppd.inc"

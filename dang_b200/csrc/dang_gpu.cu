@@ -549,6 +549,7 @@ int dang_gpu_destroy(dang_gpu_t *h) {
   if (!h) return DANG_GPU_EINVAL;
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
+  post_release(h);
   if (h->comm) g_nccl.CommDestroy(h->comm);
   for (int g = 0; g < DG_MAX_RANKS; g++)
     if (h->peer_ptr[g] && g != h->rank) cudaIpcCloseMemHandle(h->peer_ptr[g]);

@@ -123,6 +123,18 @@ struct CgGroupHost {
   int last_iter[3] = {0, 0, 0};  // iterations of the previous solve (sizes the first batch)
 };
 
+// running posterior moments of dang_gpu_posterior_*: one {mean, M2} pair per accumulated element (kernels_post.cuh)
+struct PostHost {
+  int what = 0;                 // DANG_POST_* bits fixed at _begin; 0: not begun
+  int pol_lo = 0, pol_hi = 0;   // CHI_MAP / RESIDUAL: the pol_type range of dang_gpu_get_sky_model
+  int64_t n = 0;                // samples added
+  double2 *amp[DG_MAX_COMPS] = {};             // [nmaps][Ppad], components with a map amplitude
+  double2 *idx[DG_MAX_COMPS][DG_MAXIND] = {};  // [nmaps][Ppad]
+  double2 *tamp[DG_MAX_COMPS] = {};            // [3][DG_MAX_BANDS], template / monopole / hi_fit
+  double2 *res = nullptr;                      // [nbands][nmaps][Ppad]
+  double2 *chi = nullptr;                      // [nmaps][Ppad]
+};
+
 struct KStat {
   int64_t launches = 0;
   double ms = 0, bytes = 0;
@@ -263,6 +275,8 @@ struct dang_gpu {
   int fs_cont_ic = -1, fs_cont_nind = -1, fs_cont_S = 0, fs_cont_plane0 = -1;
   uint64_t fs_cont_epoch = 0;
   bool fs_tab_written = false;   // set by sample_fullsky for dang_gpu_sample_index: table already refreshed on the device
+
+  PostHost post;  // dang_gpu_posterior_* (host_post.cu)
 
   // comm
   int nranks = 1, rank = 0;
@@ -518,6 +532,7 @@ void monopole_to_offset(dang_gpu *h, const CompHost &c);                        
 void upload_tamp(dang_gpu *h, CompHost &c);                                        // dang_gpu.cu
 void run_chisq(dang_gpu *h, int pol_lo, int pol_hi, double *sky, double *res, double *chi_map,
                double out4[4]);                                                    // host_data.cu
+void post_release(dang_gpu *h);                                                    // host_post.cu
 void mh_view(dang_gpu *h, int ic, int nind, int map_n, int nsample, int ml_mode, MhView &mh);  // host_mh_fs.cu
 void ensure_zu(dang_gpu *h, size_t n);
 void ensure_decisions(dang_gpu *h, size_t n);

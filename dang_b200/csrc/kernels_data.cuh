@@ -11,14 +11,25 @@ struct ChisqView {
   double *chi_map;    // [nmaps][Ppad] or nullptr
 };
 
-// out[0..2] = sum over unmasked pixels of chi_map(:,k) (already / nbands), out[3] = #unmasked
-template <int NC>
+// Where K6 puts what it computes per pixel: the sky model and residual t of every (band, plane), and chi_map(:,k).
+// ChisqStore writes the maps the host asked for and reduces chi-square (dang_gpu_chisq / dang_gpu_get_sky_model);
+// the posterior sink of kernels_post.cuh folds them into running moments instead.  kMaps: the sink always takes
+// the maps (every plane, every pixel, as dang_gpu_get_sky_model); kReduce: the chi-square sums go to `out`.
+struct ChisqStore {
+  static constexpr bool kMaps = false, kReduce = true;
+  __device__ __forceinline__ void sky(const ChisqView &cv, size_t off, double v) const { if (cv.sky) cv.sky[off] = v; }
+  __device__ __forceinline__ void res(const ChisqView &cv, size_t off, double v) const { if (cv.res) cv.res[off] = v; }
+  __device__ __forceinline__ void chi(const ChisqView &cv, size_t off, double v) const { if (cv.chi_map) cv.chi_map[off] = v; }
+};
+
+// K6.  out[0..2] = sum over unmasked pixels of chi_map(:,k) (already / nbands), out[3] = #unmasked (ChisqStore)
+template <int NC, class Sink = ChisqStore>
 __global__ void __launch_bounds__(DG_THREADS)
 chisq_kernel(const ModelView mv, const ChisqView cv, double *partials, unsigned int *ticket,
-             double *out) {
+             double *out, const Sink sink = Sink()) {
   __shared__ double smem[4 * 32];
   double acc[4] = {0.0, 0.0, 0.0, 0.0};
-  const bool maps = cv.sky != nullptr || cv.res != nullptr;
+  const bool maps = Sink::kMaps || cv.sky != nullptr || cv.res != nullptr;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < mv.P; p += stride) {
     const bool use = mv.mask[p] != 0;
@@ -71,8 +82,8 @@ chisq_kernel(const ModelView mv, const ChisqView cv, double *partials, unsigned 
           if (c < mv.ncomp && mv.comp[c].in_sky) sky = sky + a[k][c] * sed[k][c];  // (monopoles are offsets, :357-361)
         const double sig = ldg_stream(mv.sig + off);
         const double t = (k == 0) ? (sig - mv.offset[j]) / mv.gain[j] - sky : sig - sky;  // :384-387
-        if (cv.sky) cv.sky[off] = sky;
-        if (cv.res) cv.res[off] = t;
+        sink.sky(cv, off, sky);
+        sink.res(cv, off, t);
         if (use && k >= cv.k_lo && k <= cv.k_hi) {
           const double rms = ldg_stream(mv.rms + off);
           chi[k] = chi[k] + (t * t) / (rms * rms);  // :510-516
@@ -83,11 +94,11 @@ chisq_kernel(const ModelView mv, const ChisqView cv, double *partials, unsigned 
     for (int k = 0; k < 3; k++) {
       if (k >= mv.nmaps) continue;
       const double v = (use && k >= cv.k_lo && k <= cv.k_hi) ? chi[k] / mv.nbands : 0.0;  // :523
-      if (cv.chi_map) cv.chi_map[(size_t)k * mv.Ppad + p] = v;
+      sink.chi(cv, (size_t)k * mv.Ppad + p, v);
       acc[k] += v;
     }
   }
-  grid_reduce<4>(acc, smem, partials, ticket, out);
+  if constexpr (Sink::kReduce) grid_reduce<4>(acc, smem, partials, ticket, out);
 }
 
 // mask_avg, src/dang_util_mod.f90:186-206: out[0] = sum over unmasked of map, out[1] = count

@@ -38,6 +38,8 @@ OPT_STREAM_RING = 16
 OPT_DEFER_D2H = 17
 OPT_DEFER_SCALARS = 18
 KERNEL_COUNT = 12
+# kinds of dang_gpu_posterior_* (a bit set at posterior_begin, one bit per posterior / posterior_rhat call)
+POST_AMPLITUDE, POST_INDICES, POST_CHI_MAP, POST_RESIDUAL, POST_TEMPLATE_AMPLITUDES = 1, 2, 4, 8, 16
 
 
 class DangGpuError(RuntimeError):
@@ -429,6 +431,36 @@ class Engine:
         return dict(n_iter=n_iter.value, delta=delta.value, chisq_after_amplitudes=chi_a, accept=acc.value,
                     index_value=val.value, chisq_after_index=chi_i, chisq_amplitudes=total(chi_a), chisq_index=total(chi_i))
 
+    # ------------------------------------------------------------------ posterior summaries (not in the reference)
+    def posterior_begin(self, what: int, pol_lo: Optional[int] = None, pol_hi: Optional[int] = None):
+        """Zero running moments of the POST_* kinds in `what`; CHI_MAP / RESIDUAL are those of update_sky_model over
+        pol_lo..pol_hi (default cfg.pol_type).  The caller decides burn-in and thinning by when it accumulates."""
+        lo, hi = self.cfg.pol_type
+        self._ck(self.lib.dang_gpu_posterior_begin(self.h, int(what), lo if pol_lo is None else pol_lo,
+                                                   hi if pol_hi is None else pol_hi))
+
+    def posterior_accumulate(self):
+        """Add the current state as one sample (stream ordered, no host wait)."""
+        self._ck(self.lib.dang_gpu_posterior_accumulate(self.h))
+
+    def _posterior_shape(self, kind: int):
+        if kind == POST_RESIDUAL:
+            return (self.nbands, self.nmaps, self.npix)
+        if kind == POST_TEMPLATE_AMPLITUDES:
+            return (self.nmaps, self.nbands)
+        return (self.nmaps, self.npix)
+
+    def posterior(self, kind: int, ic: int = 0, nind: int = 0) -> Tuple[np.ndarray, np.ndarray, int]:
+        """(mean, std, n) in the shapes of amplitude / indices(ic)[nind] / update_sky_model / template_amplitudes;
+        std is NaN while n < 2.  Only this handle's pixels are written (the rest stay 0)."""
+        mean, std = np.zeros(self._posterior_shape(kind)), np.zeros(self._posterior_shape(kind))
+        n = C.c_int64()
+        self._ck(self.lib.dang_gpu_posterior_get(self.h, int(kind), ic, nind, _dp(mean), _dp(std), C.byref(n)))
+        return mean, std, n.value
+
+    def posterior_end(self):
+        self._ck(self.lib.dang_gpu_posterior_end(self.h))
+
     # ------------------------------------------------------------------ instrumentation
     def sync(self):
         self._ck(self.lib.dang_gpu_sync(self.h))
@@ -453,6 +485,18 @@ class Engine:
             self._ck(self.lib.dang_gpu_kernel_stats(self.h, k, C.byref(n), C.byref(ms), C.byref(by), int(reset)))
             out[self.lib.dang_gpu_kernel_name(k).decode()] = dict(launches=n.value, ms=ms.value, bytes=by.value)
         return out
+
+
+def posterior_rhat(engines: Sequence[Engine], kind: int, ic: int = 0, nind: int = 0) -> np.ndarray:
+    """Gelman-Rubin R-hat per element across chains (one Engine each, same device and pixel range, same samples
+    accumulated), in the shape of Engine.posterior."""
+    lib = _lib.load()
+    hs = (_lib.vp * len(engines))(*[e.h for e in engines])
+    out = np.zeros(engines[0]._posterior_shape(kind))
+    rc = lib.dang_gpu_posterior_rhat(hs, len(engines), int(kind), ic, nind, _dp(out))
+    if rc != 0:
+        raise DangGpuError(f"dang_gpu_posterior_rhat rc={rc}: {lib.dang_gpu_last_error(engines[0].h).decode()}")
+    return out
 
 
 def setup_torch_comm(eng: "Engine", mailboxes: bool = True):

@@ -30,6 +30,8 @@ module dang_gpu_mod
   public :: dang_gpu_init, dang_gpu_finalize, dang_gpu_upload_ddata
   public :: sample_cg_groups_gpu, sample_spectral_parameters_gpu, compute_chisq_gpu, sample_calibrators_gpu
   public :: dang_gpu_download_components, dang_gpu_download_sky_model
+  public :: posterior_begin_gpu, posterior_accumulate_gpu, posterior_get_gpu
+  public :: POST_AMPLITUDE, POST_INDICES, POST_CHI_MAP, POST_RESIDUAL, POST_TEMPLATE_AMPLITUDES
 
   type(c_ptr), save :: handle = c_null_ptr
   integer(i8b), save :: gpu_seed = 20260101_i8b   ! device Philox seed, advanced every draw
@@ -40,6 +42,8 @@ module dang_gpu_mod
   integer(c_int), parameter :: LNL_CHISQ = 0, LNL_MARGINAL = 1, LNL_PRIOR = 2
   integer(c_int), parameter :: PRIOR_UNIFORM = 0, PRIOR_GAUSSIAN = 1, PRIOR_JEFFREYS = 2
   integer(c_int), parameter :: ML_OPTIMIZE = 0, ML_SAMPLE = 1
+  integer(c_int), parameter :: POST_AMPLITUDE = 1, POST_INDICES = 2, POST_CHI_MAP = 4, POST_RESIDUAL = 8, &
+       POST_TEMPLATE_AMPLITUDES = 16
 
   interface
      integer(c_int) function dang_gpu_create(device, nside, npix, nmaps, nbands, ncomp, pix_lo, pix_hi, h) &
@@ -316,6 +320,34 @@ module dang_gpu_mod
        real(c_double) :: delta_final, accept, index_value
        real(c_double), intent(out) :: chisq_after_amplitudes(*), chisq_after_index(*)
      end function dang_gpu_iteration_scalars
+     ! ---- posterior summaries on the device (not in the reference): running mean / M2 of the chain state, added by
+     !      _accumulate after each iteration past burn-in; _get downloads mean and std where write_maps is due
+     integer(c_int) function dang_gpu_posterior_begin(h, what, pol_lo, pol_hi) bind(C, name='dang_gpu_posterior_begin')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: h
+       integer(c_int), value :: what, pol_lo, pol_hi
+     end function dang_gpu_posterior_begin
+     integer(c_int) function dang_gpu_posterior_accumulate(h) bind(C, name='dang_gpu_posterior_accumulate')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: h
+     end function dang_gpu_posterior_accumulate
+     integer(c_int) function dang_gpu_posterior_get(h, kind, ic, nind, mean, stddev, n) bind(C, name='dang_gpu_posterior_get')
+       import :: c_int, c_int64_t, c_double, c_ptr
+       type(c_ptr), value :: h
+       integer(c_int), value :: kind, ic, nind
+       real(c_double), intent(out) :: mean(*), stddev(*)
+       integer(c_int64_t) :: n
+     end function dang_gpu_posterior_get
+     integer(c_int) function dang_gpu_posterior_end(h) bind(C, name='dang_gpu_posterior_end')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: h
+     end function dang_gpu_posterior_end
+     integer(c_int) function dang_gpu_posterior_rhat(hs, m, kind, ic, nind, rhat) bind(C, name='dang_gpu_posterior_rhat')
+       import :: c_int, c_double, c_ptr
+       type(c_ptr), intent(in) :: hs(*)
+       integer(c_int), value :: m, kind, ic, nind
+       real(c_double), intent(out) :: rhat(*)
+     end function dang_gpu_posterior_rhat
   end interface
 
 contains
@@ -640,5 +672,27 @@ contains
          int(ddata%pol_type(size(ddata%pol_type)),c_int), ddata%sky_model, ddata%res_map, ddata%chi_map), &
          'get_sky_model')
   end subroutine dang_gpu_download_sky_model
+
+  subroutine posterior_begin_gpu(ddata, what)
+    ! zero the running moments of the POST_* kinds in `what`; CHI_MAP / RESIDUAL over ddata%pol_type
+    type(dang_data), intent(in) :: ddata
+    integer(c_int),  intent(in) :: what
+    call gpu_check(dang_gpu_posterior_begin(handle, what, int(ddata%pol_type(1),c_int), &
+         int(ddata%pol_type(size(ddata%pol_type)),c_int)), 'posterior_begin')
+  end subroutine posterior_begin_gpu
+
+  subroutine posterior_accumulate_gpu()
+    ! add the current state as one sample: stream ordered, no host wait
+    call gpu_check(dang_gpu_posterior_accumulate(handle), 'posterior_accumulate')
+  end subroutine posterior_accumulate_gpu
+
+  subroutine posterior_get_gpu(kind, ic, nind, mean, stddev, n)
+    ! mean / std of one kind, in the layout of the matching array (ic, nind: 1-based, as c%indices(:,:,nind))
+    integer(c_int),     intent(in)  :: kind, ic, nind
+    real(dp),           intent(out) :: mean(*), stddev(*)
+    integer(c_int64_t), intent(out) :: n
+    call gpu_check(dang_gpu_posterior_get(handle, kind, int(ic-1,c_int), int(nind-1,c_int), mean, stddev, n), &
+         'posterior_get')
+  end subroutine posterior_get_gpu
 
 end module dang_gpu_mod

@@ -348,6 +348,38 @@ int dang_gpu_bandpass_quadrature(double nu_c_hz, int n_bp, const double *nu0_hz,
  * more (up to n_bp / 2) where that is not enough.  Read-only. */
 int dang_gpu_band_samples(dang_gpu_t *h, int band, int *n_samples);
 
+/* ---- posterior summaries on the device.  NOT in the reference: its users set OUTPUT_ITER = 1, let write_maps write
+ * every sample and compute mean / std maps offline.  Here the chain stays resident and running moments accumulate
+ * next to it; the host downloads only the summaries, when write_maps is due (INTEGRATION.md).
+ * _begin: allocate and zero the accumulators of the kinds in `what` (a set of DANG_POST_* bits, fixed until _end or
+ *   the next _begin, which starts again from zero), n = 0.  pol_lo..pol_hi: the range dang_gpu_get_sky_model takes,
+ *   used by CHI_MAP / RESIDUAL (ignored otherwise).
+ *     AMPLITUDE            c%amplitude of every component with a map amplitude (not template / monopole / hi_fit,
+ *                          whose map is fixed, nor T_cmb, which has none)
+ *     INDICES              every index map of every component, per-pixel or full-sky
+ *     CHI_MAP, RESIDUAL    the chi_map / res_map dang_gpu_get_sky_model(h, pol_lo, pol_hi, ...) would return
+ *     TEMPLATE_AMPLITUDES  template_amplitudes of template / monopole / hi_fit components
+ * _accumulate: add the current state as one sample; stream ordered, no host wait.  Per element, n the count after
+ *   adding x, every operation rounded separately (no FMA):  d = x - mean;  mean += d / n;  M2 += d * (x - mean).
+ * _get: synchronous; mean and stddev = sqrt(M2 / (n - 1)) (NaN for n < 2; stddev may be NULL) in the layout of the
+ *   getter of that quantity: (npix,nmaps) for AMPLITUDE of component ic, INDICES of (ic, nind) and CHI_MAP,
+ *   (npix,nmaps,nbands) for RESIDUAL, (nbands,nmaps) for TEMPLATE_AMPLITUDES of ic; only this handle's pixels are
+ *   written.  ic / nind are ignored by the kinds that do not use them.
+ * _get / _accumulate / _end before _begin, or _get of a kind not begun: DANG_GPU_ESTATE; a bad ic, nind or kind:
+ *   DANG_GPU_EINVAL.  Nothing crosses ranks: each rank accumulates its own pixels.
+ * _rhat: the classic Gelman-Rubin statistic (not split-chain) per element over the m handles hs[0..m-1] (same device,
+ *   same pixel range, the kind begun and the same n >= 2 on each; otherwise DANG_GPU_EINVAL, message on hs[0]),
+ *   in _get's layout.  Sums run over the chains in the order given, each operation rounded separately:
+ *   W = (sum M2_c / (n-1)) / m,  mu = (sum mean_c) / m,  B/n = (sum (mean_c - mu)^2) / (m - 1),
+ *   R = sqrt((((n-1)/n) W + B/n) / W);  NaN where W = 0 (e.g. masked pixels of the chi-square map). */
+enum { DANG_POST_AMPLITUDE = 1, DANG_POST_INDICES = 2, DANG_POST_CHI_MAP = 4,
+       DANG_POST_RESIDUAL = 8, DANG_POST_TEMPLATE_AMPLITUDES = 16 };
+int dang_gpu_posterior_begin(dang_gpu_t *h, int what, int pol_lo, int pol_hi);
+int dang_gpu_posterior_accumulate(dang_gpu_t *h);
+int dang_gpu_posterior_get(dang_gpu_t *h, int kind, int ic, int nind, double *mean, double *stddev, int64_t *n);
+int dang_gpu_posterior_end(dang_gpu_t *h);
+int dang_gpu_posterior_rhat(dang_gpu_t *const *hs, int m, int kind, int ic, int nind, double *rhat);
+
 /* ---- instrumentation (bench.py) ---- */
 int dang_gpu_host_alloc(void **ptr, uint64_t bytes); /* pinned host memory */
 int dang_gpu_host_free(void *ptr);
