@@ -84,6 +84,8 @@ SIGNATURES = {
     "dang_gpu_posterior_get": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, c_dp, c_dp, c_i64p]),
     "dang_gpu_posterior_end": (C.c_int, [vp]),
     "dang_gpu_posterior_rhat": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, c_dp]),
+    "dang_gpu_posterior_begin_batched": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "dang_gpu_posterior_ess": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, c_dp, c_dp]),
 }
 
 _lib = None

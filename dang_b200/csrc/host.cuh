@@ -123,10 +123,12 @@ struct CgGroupHost {
   int last_iter[3] = {0, 0, 0};  // iterations of the previous solve (sizes the first batch)
 };
 
-// running posterior moments of dang_gpu_posterior_*: one {mean, M2} pair per accumulated element (kernels_post.cuh)
+// running posterior moments of dang_gpu_posterior_*: one {mean, M2} pair per accumulated element (kernels_post.cuh).
+// With batch means each allocation of L elements is [L] {mean, M2} | [L] {bmean, bM2} | [L] double bsum.
 struct PostHost {
   int what = 0;                 // DANG_POST_* bits fixed at _begin; 0: not begun
   int pol_lo = 0, pol_hi = 0;   // CHI_MAP / RESIDUAL: the pol_type range of dang_gpu_get_sky_model
+  int batch_len = 0;            // b of dang_gpu_posterior_begin_batched; 0: no batch accumulators
   int64_t n = 0;                // samples added
   double2 *amp[DG_MAX_COMPS] = {};             // [nmaps][Ppad], components with a map amplitude
   double2 *idx[DG_MAX_COMPS][DG_MAXIND] = {};  // [nmaps][Ppad]

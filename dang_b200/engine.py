@@ -432,12 +432,17 @@ class Engine:
                     index_value=val.value, chisq_after_index=chi_i, chisq_amplitudes=total(chi_a), chisq_index=total(chi_i))
 
     # ------------------------------------------------------------------ posterior summaries (not in the reference)
-    def posterior_begin(self, what: int, pol_lo: Optional[int] = None, pol_hi: Optional[int] = None):
+    def posterior_begin(self, what: int, pol_lo: Optional[int] = None, pol_hi: Optional[int] = None,
+                        batch_len: int = 0):
         """Zero running moments of the POST_* kinds in `what`; CHI_MAP / RESIDUAL are those of update_sky_model over
-        pol_lo..pol_hi (default cfg.pol_type).  The caller decides burn-in and thinning by when it accumulates."""
+        pol_lo..pol_hi (default cfg.pol_type).  The caller decides burn-in and thinning by when it accumulates.
+        batch_len > 0 also keeps batch means of batch_len consecutive samples, for posterior_ess; 0: none."""
         lo, hi = self.cfg.pol_type
-        self._ck(self.lib.dang_gpu_posterior_begin(self.h, int(what), lo if pol_lo is None else pol_lo,
-                                                   hi if pol_hi is None else pol_hi))
+        lo, hi = lo if pol_lo is None else pol_lo, hi if pol_hi is None else pol_hi
+        if batch_len:
+            self._ck(self.lib.dang_gpu_posterior_begin_batched(self.h, int(what), lo, hi, int(batch_len)))
+        else:
+            self._ck(self.lib.dang_gpu_posterior_begin(self.h, int(what), lo, hi))
 
     def posterior_accumulate(self):
         """Add the current state as one sample (stream ordered, no host wait)."""
@@ -497,6 +502,19 @@ def posterior_rhat(engines: Sequence[Engine], kind: int, ic: int = 0, nind: int 
     if rc != 0:
         raise DangGpuError(f"dang_gpu_posterior_rhat rc={rc}: {lib.dang_gpu_last_error(engines[0].h).decode()}")
     return out
+
+
+def posterior_ess(engines: Sequence[Engine], kind: int, ic: int = 0, nind: int = 0) -> Tuple[np.ndarray, np.ndarray]:
+    """(ess, mcse): batch-means effective sample size and Monte Carlo standard error of the posterior mean per
+    element, of one chain or pooled over several (one Engine each, begun with the same batch_len, same device and
+    pixel range, same samples accumulated), in the shape of Engine.posterior."""
+    lib = _lib.load()
+    hs = (_lib.vp * len(engines))(*[e.h for e in engines])
+    ess, mcse = np.zeros(engines[0]._posterior_shape(kind)), np.zeros(engines[0]._posterior_shape(kind))
+    rc = lib.dang_gpu_posterior_ess(hs, len(engines), int(kind), ic, nind, _dp(ess), _dp(mcse))
+    if rc != 0:
+        raise DangGpuError(f"dang_gpu_posterior_ess rc={rc}: {lib.dang_gpu_last_error(engines[0].h).decode()}")
+    return ess, mcse
 
 
 def setup_torch_comm(eng: "Engine", mailboxes: bool = True):

@@ -31,6 +31,7 @@ module dang_gpu_mod
   public :: sample_cg_groups_gpu, sample_spectral_parameters_gpu, compute_chisq_gpu, sample_calibrators_gpu
   public :: dang_gpu_download_components, dang_gpu_download_sky_model
   public :: posterior_begin_gpu, posterior_accumulate_gpu, posterior_get_gpu
+  public :: posterior_begin_batched_gpu, posterior_ess_gpu
   public :: POST_AMPLITUDE, POST_INDICES, POST_CHI_MAP, POST_RESIDUAL, POST_TEMPLATE_AMPLITUDES
 
   type(c_ptr), save :: handle = c_null_ptr
@@ -348,6 +349,20 @@ module dang_gpu_mod
        integer(c_int), value :: m, kind, ic, nind
        real(c_double), intent(out) :: rhat(*)
      end function dang_gpu_posterior_rhat
+     ! batch means next to the moments (b = batch_len consecutive samples), for the effective sample size and the
+     ! Monte Carlo standard error of the posterior mean
+     integer(c_int) function dang_gpu_posterior_begin_batched(h, what, pol_lo, pol_hi, batch_len) &
+          bind(C, name='dang_gpu_posterior_begin_batched')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: h
+       integer(c_int), value :: what, pol_lo, pol_hi, batch_len
+     end function dang_gpu_posterior_begin_batched
+     integer(c_int) function dang_gpu_posterior_ess(hs, m, kind, ic, nind, ess, mcse) bind(C, name='dang_gpu_posterior_ess')
+       import :: c_int, c_double, c_ptr
+       type(c_ptr), intent(in) :: hs(*)
+       integer(c_int), value :: m, kind, ic, nind
+       real(c_double), intent(out) :: ess(*), mcse(*)
+     end function dang_gpu_posterior_ess
   end interface
 
 contains
@@ -694,5 +709,25 @@ contains
     call gpu_check(dang_gpu_posterior_get(handle, kind, int(ic-1,c_int), int(nind-1,c_int), mean, stddev, n), &
          'posterior_get')
   end subroutine posterior_get_gpu
+
+  subroutine posterior_begin_batched_gpu(ddata, what, batch_len)
+    ! posterior_begin_gpu plus batch means of batch_len consecutive samples (about sqrt of the planned samples,
+    ! at least 20 batches), which posterior_ess_gpu reads
+    type(dang_data), intent(in) :: ddata
+    integer(c_int),  intent(in) :: what, batch_len
+    call gpu_check(dang_gpu_posterior_begin_batched(handle, what, int(ddata%pol_type(1),c_int), &
+         int(ddata%pol_type(size(ddata%pol_type)),c_int), batch_len), 'posterior_begin_batched')
+  end subroutine posterior_begin_batched_gpu
+
+  subroutine posterior_ess_gpu(kind, ic, nind, ess, mcse)
+    ! effective sample size and Monte Carlo standard error of the posterior mean of this chain, in the layout of
+    ! posterior_get_gpu (ic, nind: 1-based)
+    integer(c_int), intent(in)  :: kind, ic, nind
+    real(dp),       intent(out) :: ess(*), mcse(*)
+    type(c_ptr) :: hs(1)
+    hs(1) = handle
+    call gpu_check(dang_gpu_posterior_ess(hs, 1_c_int, kind, int(ic-1,c_int), int(nind-1,c_int), ess, mcse), &
+         'posterior_ess')
+  end subroutine posterior_ess_gpu
 
 end module dang_gpu_mod

@@ -371,14 +371,33 @@ int dang_gpu_band_samples(dang_gpu_t *h, int band, int *n_samples);
  *   same pixel range, the kind begun and the same n >= 2 on each; otherwise DANG_GPU_EINVAL, message on hs[0]),
  *   in _get's layout.  Sums run over the chains in the order given, each operation rounded separately:
  *   W = (sum M2_c / (n-1)) / m,  mu = (sum mean_c) / m,  B/n = (sum (mean_c - mu)^2) / (m - 1),
- *   R = sqrt((((n-1)/n) W + B/n) / W);  NaN where W = 0 (e.g. masked pixels of the chi-square map). */
+ *   R = sqrt((((n-1)/n) W + B/n) / W);  NaN where W = 0 (e.g. masked pixels of the chi-square map).
+ * _begin_batched: _begin plus batch-means accumulators for every kind in `what` (24 more bytes per element), so
+ *   that _ess can estimate how many independent samples the mean rests on.  batch_len = b >= 1, else
+ *   DANG_GPU_EINVAL.  _accumulate, _get, _end and _rhat behave as after _begin (_get returns the same mean and
+ *   stddev bit for bit).  Sample n at position j = ((n-1) mod b) + 1 of its batch, each operation rounded separately:
+ *   {mean, M2} as above;  bsum = (j == 1) ? x : bsum + x;  if j == b:  k = n / b,  y = bsum / b,  d = y - bmean,
+ *   bmean += d / k,  bM2 += d * (y - bmean).  A partial batch at the end is left out of {bmean, bM2}.
+ * _ess: batch-means effective sample size and Monte Carlo standard error of the posterior mean per element, over
+ *   m >= 1 handles hs[0..m-1] (m = 1: one chain; m > 1 pools the chains), in _get's layout; ess or mcse may be
+ *   NULL, not both.  Synchronous.  Every handle needs the same device and pixel range, the kind begun batched, the
+ *   same n and b, and K = n / b >= 2 complete batches; otherwise DANG_GPU_EINVAL, message on hs[0].  A handle not
+ *   begun, or begun without batches: DANG_GPU_ESTATE.  Sums run over the chains in the order given:
+ *     mu  = (sum mean_c) / m,   A  = sum M2_c,   D  = sum (mean_c - mu) (mean_c - mu),    s2   = (A + n D) / (m n - 1)
+ *     mub = (sum bmean_c) / m,  Ab = sum bM2_c,  Db = sum (bmean_c - mub) (bmean_c - mub), sig2 = b (Ab + K Db) / (m K - 1)
+ *     ess = (m n) s2 / sig2,    mcse = sqrt(sig2 / (m n));  both NaN where sig2 = 0.
+ *   sig2 estimates the asymptotic variance of the chain mean (Flegal & Jones 2010).  For m > 1, chains that
+ *   disagree inflate Db and the ESS collapses.  ESS is not capped at m n.  Choose b near sqrt(planned n), with
+ *   K >= 20 for a stable estimate; the library does not choose b. */
 enum { DANG_POST_AMPLITUDE = 1, DANG_POST_INDICES = 2, DANG_POST_CHI_MAP = 4,
        DANG_POST_RESIDUAL = 8, DANG_POST_TEMPLATE_AMPLITUDES = 16 };
 int dang_gpu_posterior_begin(dang_gpu_t *h, int what, int pol_lo, int pol_hi);
+int dang_gpu_posterior_begin_batched(dang_gpu_t *h, int what, int pol_lo, int pol_hi, int batch_len);
 int dang_gpu_posterior_accumulate(dang_gpu_t *h);
 int dang_gpu_posterior_get(dang_gpu_t *h, int kind, int ic, int nind, double *mean, double *stddev, int64_t *n);
 int dang_gpu_posterior_end(dang_gpu_t *h);
 int dang_gpu_posterior_rhat(dang_gpu_t *const *hs, int m, int kind, int ic, int nind, double *rhat);
+int dang_gpu_posterior_ess(dang_gpu_t *const *hs, int m, int kind, int ic, int nind, double *ess, double *mcse);
 
 /* ---- instrumentation (bench.py) ---- */
 int dang_gpu_host_alloc(void **ptr, uint64_t bytes); /* pinned host memory */
